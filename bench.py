@@ -8,6 +8,8 @@ A "step" is one pass of the fused kernel over that batch.  N>1: every rank owns 
 (weak scaling, streams are independent units) and the per-chunk probabilities are all-gathered over NCCL.
 
   python bench.py --gpus 1 --steps 20 --warmup 3            own arm  (GPU, device-resident inputs + e2e)
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's probabilities to DIR/probs.npy
+                                                            (seeded inputs: the same arguments give the same inputs on every run)
   python bench.py --impl reference ...                      reference arm: the UNMODIFIED reference (baseline/_ref, TorchScript
                                                             model, audio_forward) on the host cores
 
@@ -61,7 +63,30 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the sustained / latency / segment / configs[3] legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path,
+                    help="write the probabilities of the last timed step to DIR/probs.npy (float32) for output-by-output comparison of builds")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU arm computed (--impl b200)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 63 * 10**6     # --dump-outputs writes at most 64 MB in all, .npy headers included
+
+
+def dump_outputs(out_dir, probs):
+    """probs: float32 numpy [rows, T].  Above DUMP_LIMIT_BYTES a fixed, seeded sample of rows is written, and the row indices beside it
+    (probs_rows.npy, float64), so that two runs with the same arguments write the same sample."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    probs = np.ascontiguousarray(probs, np.float32)
+    max_rows = max(1, DUMP_LIMIT_BYTES // (probs.shape[1] * 4 + 8))
+    if probs.shape[0] > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(probs.shape[0], max_rows, replace=False))
+        np.save(out_dir / "probs_rows.npy", rows.astype(np.float64))
+        probs = probs[rows]
+    np.save(out_dir / "probs.npy", probs)
 
 
 def peaks():
@@ -399,6 +424,9 @@ def run_b200(args):
         ref = torch.zeros(world, device=dev, dtype=torch.float64); ref[rank] = probs[last].sum(dtype=torch.float64)
         dist.all_reduce(ref)
         assert torch.equal(chk, ref), "gathered blocks differ from the owners' results"
+    if args.dump_outputs and rank == 0:
+        last = (args.steps - 1) & 1
+        dump_outputs(args.dump_outputs, (gathered if world > 1 else probs)[last].cpu().numpy())
     chunks_per_step = B * T * world
     value = chunks_per_step * args.steps / (ms_total * 1e-3)
 

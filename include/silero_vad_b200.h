@@ -160,6 +160,39 @@ int svad_collect_chunks_device(svad_engine* e, const void* d_wav, int elem_bytes
                                const int64_t* seg_rows, const int64_t* seg_bounds, int64_t n_seg, int drop, void* d_out,
                                int64_t out_cap, int64_t* out_offsets, void* stream);
 
+/* ---- decoder fine-tuning --------------------------------------------------------------------------------------------------------
+ * The encoder is frozen; the decoder (LSTMCell(128 -> 128) + Dropout -> ReLU -> Conv1d(128 -> 1) -> Sigmoid) is trained on the
+ * encoder's outputs.  All pointers are device memory of the engine's device unless noted; work is enqueued on `stream`.
+ *
+ * Encoder features: d_audio f32 [B][ld], L valid samples per row, L a multiple of the chunk size n (512 @16 kHz, 256 @8 kHz);
+ * d_ctx_in [B][n/8] (or NULL = zeros) are the samples that precede each row; d_feat f32 [B][L/n][128] receives the post-ReLU
+ * encoder output (the LSTM input) of every chunk.  Always the fp32 tile kernel, whatever svad_engine_set_kernel selected. */
+int svad_features_device(svad_engine* e, int sr, int B, int64_t L, int64_t ld, const float* d_audio, const float* d_ctx_in,
+                         float* d_feat, void* stream);
+/* Decoder scans over B streams x T steps from zero state.  Parameters in torch layout: W_ih, W_hh [512][128], b_ih, b_hh [512],
+ * w_head [128], b_head [1]; gate order i, f, g, o.  d_drop [B][T][128] (or NULL) multiplies h on the head path only.
+ * svad_decoder_tape_floats: floats of the tape the forward pass saves for the backward pass (activated gates and c);
+ * svad_decoder_workspace_bytes: scratch of the forward (backward = 0) or backward (backward = 1) pass.  Both return SVAD_EINVAL
+ * for negative sizes. */
+int64_t svad_decoder_tape_floats(int B, int64_t T);
+int64_t svad_decoder_workspace_bytes(int B, int64_t T, int backward);
+/* d_feat [B][T][128] -> d_probs [B][T]; d_tape (or NULL when no backward pass follows) receives svad_decoder_tape_floats floats. */
+int svad_decoder_forward_device(svad_engine* e, int B, int64_t T, const float* d_feat, const float* d_w_ih, const float* d_w_hh,
+                                const float* d_b_ih, const float* d_b_hh, const float* d_w_head, const float* d_b_head,
+                                const float* d_drop, float* d_probs, float* d_tape, void* d_work, void* stream);
+/* d_dprobs [B][T] = dloss / dprobs -> dW_ih, dW_hh [512][128], db [512] (the gradient of b_ih and of b_hh alike), dw_head [128],
+ * db_head [1].  d_probs and d_tape are what the forward pass with the same parameters and d_drop produced.  Fixed-order
+ * reductions: the result does not change from call to call. */
+int svad_decoder_backward_device(svad_engine* e, int B, int64_t T, const float* d_feat, const float* d_w_hh, const float* d_w_head,
+                                 const float* d_drop, const float* d_probs, const float* d_dprobs, const float* d_tape, void* d_work,
+                                 float* d_dw_ih, float* d_dw_hh, float* d_db, float* d_dw_head, float* d_db_head, void* stream);
+/* Threshold search: file f holds d_probs / d_targets [d_offsets[f], d_offsets[f+1]) (d_offsets int64 [files+1]); d_grid f64 [20]
+ * are the candidate thresholds.  For each of the 190 pairs (enter index a, exit index e < a; a outer, e inner) the hysteresis
+ * decision (p >= enter -> 1, else p <= exit -> 0, else hold; from 0) is compared with the target, in double precision;
+ * d_counts int64 [files][190] receives the number of matching chunks.  Runs on the current device. */
+int svad_threshold_grid_device(const float* d_probs, const float* d_targets, const int64_t* d_offsets, int64_t files,
+                               const double* d_grid, int64_t* d_counts, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -15,7 +15,9 @@ EXPORTS = ["svad_abi_version", "svad_last_error", "svad_engine_create", "svad_en
            "svad_forward_device", "svad_forward_device_pcm16", "svad_forward_device_ex", "svad_step_device", "svad_forward_host",
            "svad_collect_chunks_device", "svad_stream_open", "svad_stream_push", "svad_stream_reset", "svad_stream_close",
            "svad_forward_host_pcm16", "svad_step_host",
-           "svad_segment_params_default", "svad_speech_segments"]
+           "svad_segment_params_default", "svad_speech_segments",
+           "svad_features_device", "svad_decoder_tape_floats", "svad_decoder_workspace_bytes", "svad_decoder_forward_device",
+           "svad_decoder_backward_device", "svad_threshold_grid_device"]
 
 
 class SvadError(RuntimeError):
@@ -67,6 +69,14 @@ def lib():
     L.svad_segment_params_default.argtypes = [ctypes.POINTER(SegmentParams)]
     L.svad_segment_params_default.restype = None
     L.svad_speech_segments.argtypes = [vp, i64, i64, i64, vp, ctypes.POINTER(SegmentParams), vp, vp, i64, ctypes.POINTER(i64)]
+    L.svad_features_device.argtypes = [vp, i32, i32, i64, i64, vp, vp, vp, vp]
+    L.svad_decoder_tape_floats.argtypes = [i32, i64]
+    L.svad_decoder_tape_floats.restype = i64
+    L.svad_decoder_workspace_bytes.argtypes = [i32, i64, i32]
+    L.svad_decoder_workspace_bytes.restype = i64
+    L.svad_decoder_forward_device.argtypes = [vp, i32, i64] + [vp] * 12
+    L.svad_decoder_backward_device.argtypes = [vp, i32, i64] + [vp] * 14
+    L.svad_threshold_grid_device.argtypes = [vp, vp, vp, i64, vp, vp, vp]
     for name in EXPORTS:
         getattr(L, name)
     _lib = L
@@ -166,6 +176,17 @@ class Engine:
 
     def step_device(self, sr, B, x1, state_in, prob, state_out, stream=0):
         check(lib().svad_step_device(self._h, sr, B, x1, state_in, prob, state_out, stream))
+
+    # ---- decoder fine-tuning (silero_vad_b200.tuning)
+    def features_device(self, sr, B, L, ld, audio, ctx_in, feat, stream=0):
+        check(lib().svad_features_device(self._h, sr, B, L, ld, audio, ctx_in, feat, stream))
+
+    def decoder_forward_device(self, B, T, feat, w_ih, w_hh, b_ih, b_hh, w_head, b_head, drop, probs, tape, work, stream=0):
+        check(lib().svad_decoder_forward_device(self._h, B, T, feat, w_ih, w_hh, b_ih, b_hh, w_head, b_head, drop, probs, tape, work, stream))
+
+    def decoder_backward_device(self, B, T, feat, w_hh, w_head, drop, probs, dprobs, tape, work, dw_ih, dw_hh, db, dw_head, db_head, stream=0):
+        check(lib().svad_decoder_backward_device(self._h, B, T, feat, w_hh, w_head, drop, probs, dprobs, tape, work, dw_ih, dw_hh, db,
+                                                 dw_head, db_head, stream))
 
     def forward_host(self, sr, B, L, ld, audio, state_in, ctx_in, state_out, ctx_out, probs, ldp):
         check(lib().svad_forward_host(self._h, sr, B, L, ld, audio, state_in, ctx_in, state_out, ctx_out, probs, ldp))

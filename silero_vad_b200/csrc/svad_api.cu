@@ -24,6 +24,7 @@
 #include "svad_tc.h"
 #include "svad_small.h"
 #include "svad_h16.cuh"
+#include "svad_train.cuh"
 
 using namespace svad;
 
@@ -32,8 +33,9 @@ namespace {
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-template <bool SR16>
+template <bool SR16, bool FEAT = false>
 struct GpuEnv {
+    static constexpr int kNslab = FEAT ? Geo<SR16>::nslab_enc : Geo<SR16>::nslab;   // slabs per step (run_cta's FEAT)
     float* sm;
     uint64_t* full;   // [kStages] "slab landed" mbarriers (TMA transaction count)
     uint64_t* empty;  // [kStages] "slab consumed" mbarriers (one arrival per warp)
@@ -44,7 +46,7 @@ struct GpuEnv {
     __device__ __forceinline__ void sync() { __syncthreads(); }
     __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
     __device__ __forceinline__ void issue(long it) {  // one thread
-        const int idx = (int)(it % Geo<SR16>::nslab), stage = (int)(it % kStages);
+        const int idx = (int)(it % kNslab), stage = (int)(it % kStages);
         const uint32_t bytes = (uint32_t)Tape<SR16>::slab_len(idx) * 4u;
         const uint32_t bar = smem_u32(full + stage);
         const uint32_t dst = smem_u32(sm + SmemMap::stage + stage * SmemMap::stage_floats);
@@ -86,13 +88,13 @@ struct GpuEnv {
 
 constexpr size_t kSmemBytes = (size_t)SmemMap::total_floats * 4 + 64;
 
-template <bool SR16, int RM, typename S>
+template <bool SR16, int RM, typename S, bool FEAT = false>
 __global__ void __launch_bounds__(kThreads, 1) svad_fused_fp32(TileArgs a, int ntiles) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     float* sm = reinterpret_cast<float*>(smem_raw);
     uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)SmemMap::total_floats * 4);
     uint64_t* empty = full + kStages;
-    GpuEnv<SR16> env{sm, full, empty, a.tape, (int)threadIdx.x};
+    GpuEnv<SR16, FEAT> env{sm, full, empty, a.tape, (int)threadIdx.x};
     int my_tiles = 0;
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) my_tiles++;
     if (threadIdx.x == 0) {
@@ -102,11 +104,11 @@ __global__ void __launch_bounds__(kThreads, 1) svad_fused_fp32(TileArgs a, int n
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        const long total = (long)my_tiles * a.T * Geo<SR16>::nslab;
+        const long total = (long)my_tiles * a.T * GpuEnv<SR16, FEAT>::kNslab;
         for (long i = 0; i < kStages && i < total; i++) env.issue(i);
     }
     __syncthreads();
-    run_cta<SR16, RM, S>(env, a, (int)blockIdx.x, (int)gridDim.x, ntiles);
+    run_cta<SR16, RM, S, FEAT>(env, a, (int)blockIdx.x, (int)gridDim.x, ntiles);
 }
 
 
@@ -818,9 +820,9 @@ extern "C" int svad_engine_set_small_batch_max(svad_engine* e, int streams) {
 extern "C" int svad_engine_sm_count(const svad_engine* e) { return e ? e->sms : 0; }
 extern "C" int64_t svad_engine_launch_count(const svad_engine* e) { return e ? e->launches : 0; }
 
-template <bool SR16, int RM, typename S>
+template <bool SR16, int RM, typename S, bool FEAT = false>
 static int launch(svad_engine* e, const TileArgs& a, cudaStream_t st) {
-    auto kern = svad_fused_fp32<SR16, RM, S>;
+    auto kern = svad_fused_fp32<SR16, RM, S, FEAT>;
     static bool configured[16] = {};  // per device
     if (!configured[e->device & 15]) {
         CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
@@ -1374,5 +1376,149 @@ extern "C" int svad_stream_push(svad_stream* s, const float* chunk, float* prob)
     std::atomic_thread_fence(std::memory_order_acquire);
     for (int i = 0; i < s->ns; i++) prob[i] = s->out[slot * kSmallNS + i];
     s->seq++;
+    return SVAD_OK;
+}
+
+// ------------------------------------------------------------------------------------------ decoder fine-tuning
+// Encoder features: the fp32 tile kernel in features mode, whatever set_kernel / set_small_batch_max say (the inference kernels
+// never hold the post-ReLU enc3 rows in fp32).
+template <bool SR16>
+static int launch_features(svad_engine* e, const TileArgs& a, cudaStream_t st) {
+    switch (pick_rows(e, a.B)) {
+        case 4: return launch<SR16, 4, float, true>(e, a, st);
+        case 5: return launch<SR16, 5, float, true>(e, a, st);
+        case 6: return launch<SR16, 6, float, true>(e, a, st);
+        case 7: return launch<SR16, 7, float, true>(e, a, st);
+        default: return launch<SR16, 8, float, true>(e, a, st);
+    }
+}
+
+extern "C" int svad_features_device(svad_engine* e, int sr, int B, int64_t L, int64_t ld, const float* d_audio, const float* d_ctx_in,
+                                    float* d_feat, void* stream) {
+    if (!e) return fail(SVAD_EINVAL, "null engine");
+    if (sr != 16000 && sr != 8000) return fail(SVAD_EINVAL, "Supported sampling rates: [8000, 16000] (got %d)", sr);
+    const int n = sr == 16000 ? 512 : 256;
+    if (B < 0 || L < 0 || L % n) return fail(SVAD_EINVAL, "features: B >= 0 and L a multiple of %d samples required (got B=%d, L=%lld)", n, B, (long long)L);
+    if (B == 0 || L == 0) return SVAD_OK;
+    if (!d_audio || !d_feat || ld < L) return fail(SVAD_EINVAL, "bad audio/feature pointer or stride");
+    CUDA_TRY(cudaSetDevice(e->device));
+    const int br = sr == 16000 ? 0 : 1;
+    TileArgs a{};
+    a.audio = d_audio; a.ld = ld; a.L = L; a.dec = 1; a.B = B; a.T = L / n;
+    a.ctx_in = d_ctx_in; a.ctx_ld = sr == 16000 ? 64 : 32;
+    a.probs = d_feat; a.ldp = a.T;   // features mode: [B][T][128]
+    a.tape = e->d_tape[br]; a.consts = e->d_consts[br];
+    return sr == 16000 ? launch_features<true>(e, a, (cudaStream_t)stream) : launch_features<false>(e, a, (cudaStream_t)stream);
+}
+
+// streams per CTA of the scans: one while the streams fit on the SMs, then 2 or 4 (a CTA's step costs little more for 4 streams)
+static int dec_group(const svad_engine* e, int B) { return B <= e->sms ? 1 : (B <= 2 * e->sms ? 2 : 4); }
+static long dec_chunks(long N) { return (N + kWgChunk - 1) / kWgChunk; }
+
+extern "C" int64_t svad_decoder_tape_floats(int B, int64_t T) { return (B < 0 || T < 0) ? SVAD_EINVAL : (int64_t)B * T * (kGates + kHid); }
+
+extern "C" int64_t svad_decoder_workspace_bytes(int B, int64_t T, int backward) {
+    if (B < 0 || T < 0) return SVAD_EINVAL;
+    const long N = (long)B * T;
+    if (!backward) return (int64_t)N * kGates * 4;   // Gx
+    return ((int64_t)N * kGates + (int64_t)B * (kHid + 1) + (int64_t)dec_chunks(N) * kGates * (2 * kHid + 1)) * 4;
+}
+
+template <class K>
+static int dec_configure(svad_engine* e, K kern, size_t smem, bool* configured) {
+    if (!configured[e->device & 15]) {
+        CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        configured[e->device & 15] = true;
+    }
+    return SVAD_OK;
+}
+
+template <int G>
+static int dec_forward(svad_engine* e, int B, long T, const float* w_hh, const float* w_head, const float* b_head, const float* drop, float* probs,
+                       float* tape, const float* gx, cudaStream_t st) {
+    static bool configured[16] = {};
+    auto kern = dec_fwd<G>;
+    if (int rc = dec_configure(e, kern, dec_fwd_smem_bytes<G>(), configured)) return rc;
+    float* tg = tape;
+    float* tc = tape ? tape + (long)B * T * kGates : nullptr;
+    kern<<<(B + G - 1) / G, kDecThreads, dec_fwd_smem_bytes<G>(), st>>>(gx, w_hh, w_head, b_head, drop, probs, tg, tc, B, T);
+    CUDA_TRY(cudaGetLastError());
+    e->launches++;
+    return SVAD_OK;
+}
+
+template <int G>
+static int dec_backward(svad_engine* e, int B, long T, const float* w_hh, const float* w_head, const float* drop, const float* probs,
+                        const float* dprobs, const float* tape, float* dgates, float* head_part, cudaStream_t st) {
+    static bool configured[16] = {};
+    auto kern = dec_bwd<G>;
+    if (int rc = dec_configure(e, kern, dec_bwd_smem_bytes<G>(), configured)) return rc;
+    kern<<<(B + G - 1) / G, kDecThreads, dec_bwd_smem_bytes<G>(), st>>>(w_hh, w_head, drop, probs, dprobs, tape, tape + (long)B * T * kGates,
+                                                                    dgates, head_part, B, T);
+    CUDA_TRY(cudaGetLastError());
+    e->launches++;
+    return SVAD_OK;
+}
+
+extern "C" int svad_decoder_forward_device(svad_engine* e, int B, int64_t T, const float* d_feat, const float* d_w_ih, const float* d_w_hh,
+                                           const float* d_b_ih, const float* d_b_hh, const float* d_w_head, const float* d_b_head,
+                                           const float* d_drop, float* d_probs, float* d_tape, void* d_work, void* stream) {
+    if (!e) return fail(SVAD_EINVAL, "null engine");
+    if (B < 0 || T < 0) return fail(SVAD_EINVAL, "negative size");
+    if (B == 0 || T == 0) return SVAD_OK;
+    if (!d_feat || !d_w_ih || !d_w_hh || !d_b_ih || !d_b_hh || !d_w_head || !d_b_head || !d_probs || !d_work)
+        return fail(SVAD_EINVAL, "null feature, parameter, probability or workspace pointer");
+    CUDA_TRY(cudaSetDevice(e->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    const long N = (long)B * T;
+    float* gx = static_cast<float*>(d_work);
+    dec_inproj<<<dim3((unsigned)((N + 63) / 64), kGates / 64), 256, 0, st>>>(d_feat, d_w_ih, d_b_ih, d_b_hh, gx, N);
+    CUDA_TRY(cudaGetLastError());
+    e->launches++;
+    switch (dec_group(e, B)) {
+        case 1: return dec_forward<1>(e, B, T, d_w_hh, d_w_head, d_b_head, d_drop, d_probs, d_tape, gx, st);
+        case 2: return dec_forward<2>(e, B, T, d_w_hh, d_w_head, d_b_head, d_drop, d_probs, d_tape, gx, st);
+        default: return dec_forward<4>(e, B, T, d_w_hh, d_w_head, d_b_head, d_drop, d_probs, d_tape, gx, st);
+    }
+}
+
+extern "C" int svad_decoder_backward_device(svad_engine* e, int B, int64_t T, const float* d_feat, const float* d_w_hh, const float* d_w_head,
+                                            const float* d_drop, const float* d_probs, const float* d_dprobs, const float* d_tape, void* d_work,
+                                            float* d_dw_ih, float* d_dw_hh, float* d_db, float* d_dw_head, float* d_db_head, void* stream) {
+    if (!e) return fail(SVAD_EINVAL, "null engine");
+    if (B < 1 || T < 1) return fail(SVAD_EINVAL, "backward needs B >= 1 and T >= 1 (got B=%d, T=%lld)", B, (long long)T);
+    if (!d_feat || !d_w_hh || !d_w_head || !d_probs || !d_dprobs || !d_tape || !d_work || !d_dw_ih || !d_dw_hh || !d_db || !d_dw_head || !d_db_head)
+        return fail(SVAD_EINVAL, "null pointer argument");
+    CUDA_TRY(cudaSetDevice(e->device));
+    const cudaStream_t st = (cudaStream_t)stream;
+    const long N = (long)B * T, nch = dec_chunks(N);
+    if (nch > 65535) return fail(SVAD_EINVAL, "backward: at most %ld steps in total", 65535L * kWgChunk);
+    float* dgates = static_cast<float*>(d_work);
+    float* head_part = dgates + N * kGates;
+    float* wg_part = head_part + (long)B * (kHid + 1);
+    int rc;
+    switch (dec_group(e, B)) {
+        case 1: rc = dec_backward<1>(e, B, T, d_w_hh, d_w_head, d_drop, d_probs, d_dprobs, d_tape, dgates, head_part, st); break;
+        case 2: rc = dec_backward<2>(e, B, T, d_w_hh, d_w_head, d_drop, d_probs, d_dprobs, d_tape, dgates, head_part, st); break;
+        default: rc = dec_backward<4>(e, B, T, d_w_hh, d_w_head, d_drop, d_probs, d_dprobs, d_tape, dgates, head_part, st); break;
+    }
+    if (rc) return rc;
+    dec_wgrad<<<dim3(kGates / 64, 2 * kHid / 64, (unsigned)nch), 256, 0, st>>>(dgates, d_feat, d_tape, d_tape + N * kGates, wg_part, T, N);
+    CUDA_TRY(cudaGetLastError());
+    const int tot = kGates * (2 * kHid + 1) + kHid + 1;
+    dec_reduce<<<(tot + 255) / 256, 256, 0, st>>>(wg_part, (int)nch, head_part, B, d_dw_ih, d_dw_hh, d_db, d_dw_head, d_db_head);
+    CUDA_TRY(cudaGetLastError());
+    e->launches += 2;
+    return SVAD_OK;
+}
+
+extern "C" int svad_threshold_grid_device(const float* d_probs, const float* d_targets, const int64_t* d_offsets, int64_t files,
+                                          const double* d_grid, int64_t* d_counts, void* stream) {
+    if (files < 0 || files > 0x7fffffff) return fail(SVAD_EINVAL, "files out of range (got %lld)", (long long)files);
+    if (files == 0) return SVAD_OK;
+    if (!d_probs || !d_targets || !d_offsets || !d_grid || !d_counts) return fail(SVAD_EINVAL, "null pointer argument");
+    threshold_grid<<<(unsigned)files, 192, 0, (cudaStream_t)stream>>>(d_probs, d_targets, reinterpret_cast<const long long*>(d_offsets), d_grid,
+                                                                    reinterpret_cast<long long*>(d_counts));
+    CUDA_TRY(cudaGetLastError());
     return SVAD_OK;
 }

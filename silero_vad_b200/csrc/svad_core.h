@@ -72,6 +72,7 @@ struct Geo {
     static constexpr int e0_nslab = SR16 ? 7 : 4;
     static constexpr int e0_cps = SR16 ? 19 : 17;  // max channels per slab (<= 21)
     static constexpr int nslab = e0_nslab + 4 + 1 + 1 + 16;
+    static constexpr int nslab_enc = nslab - 16;   // features mode: the encoder slabs only (the tape's first nslab_enc slabs)
 };
 
 // ---------------------------------------------------------------- shared-memory map (float offsets)

@@ -34,9 +34,15 @@ struct TileArgs {
     long long* dbg;         // optional: per-phase clock64 stamps of CTA 0 (tensor-core kernel, profiling builds)
 };
 
-template <bool SR16, int RM, typename S, class Env>
+// FEAT: features mode (encoder-feature export for decoder fine-tuning).  The step ends after enc3: its rows go to a.probs, which
+// then holds [B][ldp][128] floats (the post-ReLU enc3 output of chunk t of stream g, i.e. the LSTM input, at row g * ldp + t), and
+// the LSTM, the head and the state / context write-back are skipped.  (TileArgs keeps its layout: a field added for this mode
+// changed the register allocation of the inference instantiations.)  The tape walk then has G::nslab_enc slabs per step (the
+// LSTM slabs are never issued), so Env must be instantiated with the same FEAT.
+template <bool SR16, int RM, typename S, bool FEAT = false, class Env>
 SVAD_HD void run_cta(Env& env, const TileArgs& a, int first_tile, int tile_stride, int ntiles) {
     using G = Geo<SR16>;
+    constexpr int kNslab = FEAT ? G::nslab_enc : G::nslab;
     using TP = Tape<SR16>;
     const Tc tc(env.tid());
     float* sm = env.smem();
@@ -62,7 +68,7 @@ SVAD_HD void run_cta(Env& env, const TileArgs& a, int first_tile, int tile_strid
     }
     int my_tiles = 0;
     for (int tile = first_tile; tile < ntiles; tile += tile_stride) my_tiles++;
-    const long total_slabs = (long)my_tiles * a.T * G::nslab;
+    const long total_slabs = (long)my_tiles * a.T * kNslab;
     long it = 0;  // running slab counter of this CTA
 
     for (int tile = first_tile; tile < ntiles; tile += tile_stride) {
@@ -164,6 +170,17 @@ SVAD_HD void run_cta(Env& env, const TileArgs& a, int first_tile, int tile_strid
                 env.sync();
                 it++;
             }
+            if constexpr (FEAT) {
+                for (int i = tc.tid; i < kHid * kSlots; i += kThreads) {   // consecutive threads: consecutive channels of one slot
+                    const int s = i >> 7, j = i & (kHid - 1);
+                    const int g = g0 + slot_to_local<RM>(s);
+                    if (slot_valid<RM>(s) && g < a.B) a.probs[((long)g * a.ldp + t) * kHid + j] = sm[SmemMap::e3 + j * kSlots + swz_slot(s, key_hi(j))];
+                }
+                env.sync();   // e3 is read before the next step's STFT overwrites the region
+                if (t + 1 < a.T)
+                    stft_load<SR16, S>(tc.tid, 0, aud[0], cxp[0], a.L, t + 1, ((t + 2) * G::n <= a.L) && a.dec == 1, xa, xb, a.dec);
+                continue;
+            }
             // ---------------- LSTM + head
             lstm_init<RM>(tc, sm, rg);
 #pragma unroll 1
@@ -184,6 +201,7 @@ SVAD_HD void run_cta(Env& env, const TileArgs& a, int first_tile, int tile_strid
         }
         // ---- tile exit: carry state / context out
         env.sync();
+        if (FEAT) continue;
         if (a.state_out) {
             for (int i = tc.tid; i < kHid * kSlots; i += kThreads) {
                 const int s = i & 31, j = i >> 5;

@@ -29,7 +29,8 @@ class SileroVADB200:
         if device is None:
             device = torch.cuda.current_device()
         self.device = torch.device("cuda", device if isinstance(device, int) else torch.device(device).index or 0)
-        self.engine = _cabi.Engine(weights or WEIGHTS, self.device.index)
+        self.weights = Path(weights or WEIGHTS)   # the SVADW001 container the engine was built from (stock or save_tuned output)
+        self.engine = _cabi.Engine(self.weights, self.device.index)
         self.reset_states()
 
     # ------------------------------------------------------------------ reference surface

@@ -5,32 +5,19 @@ Runs only in the build container (needs /root/reference).  The only trusted weig
 source is `src/silero_vad/data/silero_vad.jit` (SURVEY.md F6); its `state_dict()`
 holds 30 fp32 tensors (15 per sample-rate branch).
 
-Outputs (raw little-endian fp32, "SVADW001" container, see `write_container`):
+Outputs (raw little-endian fp32, "SVADW001" container, see silero_vad_b200.tuning.write_container):
   silero_vad_b200/data/silero_vad_v6.weights   28 tensors (no STFT bases) - product
   oracle/data/stft_basis.weights                2 tensors (STFT conv bases) - oracle only
 """
-import struct
 import sys
 from pathlib import Path
 
 import torch
 
 REPO = Path(__file__).resolve().parents[1]
+sys.path.insert(0, str(REPO))
+from silero_vad_b200.tuning import write_container  # noqa: E402  (the one SVADW001 writer)
 JIT = Path("/root/reference/src/silero_vad/data/silero_vad.jit")
-
-
-def write_container(path: Path, tensors):
-    """magic[8] | u32 n | n x { u32 name_len | name | u32 ndim | u32 dims[ndim] | f32 data }"""
-    with open(path, "wb") as f:
-        f.write(b"SVADW001")
-        f.write(struct.pack("<I", len(tensors)))
-        for name, t in tensors:
-            nb = name.encode()
-            f.write(struct.pack("<I", len(nb)))
-            f.write(nb)
-            f.write(struct.pack("<I", t.dim()))
-            f.write(struct.pack("<%dI" % t.dim(), *t.shape))
-            f.write(t.contiguous().numpy().astype("<f4").tobytes())
 
 
 def main():
